@@ -172,6 +172,27 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_FRAMES = 2048
+
+
+def dump_outputs(dirname, ctx, res, n_frames, rank):
+    """What a caller of the timed path receives from one step: the decoded bytes and the (offset, length) of every frame in
+    them.  The bytes of a fixed, seeded sample of DUMP_FRAMES frames are written (float32, 32 MiB), the segment table in
+    full (float64, exact for offsets below 2**53), so that two builds can be compared output for output."""
+    import ctypes as C
+    L = ctx.L
+    seg = np.ctypeslib.as_array(C.cast(L.zb200_result_segments(res), C.POINTER(C.c_uint64)), shape=(n_frames, 2)).copy()
+    data = np.empty(int(L.zb200_result_size(res)), dtype=np.uint8)
+    ctx.check(L.zb200_memcpy_d2h(ctx.h, data.ctypes.data, L.zb200_result_data(res), len(data)), "d2h")
+    pick = np.sort(np.random.default_rng(0).choice(n_frames, min(n_frames, DUMP_FRAMES), replace=False))
+    sample = np.concatenate([data[int(seg[i, 0]):int(seg[i, 0] + seg[i, 1])] for i in pick])
+    suffix = "" if rank == 0 else "_rank%d" % rank
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "decompressed_sample%s.npy" % suffix), sample.astype(np.float32))
+    np.save(os.path.join(dirname, "sample_frames%s.npy" % suffix), pick.astype(np.float64))
+    np.save(os.path.join(dirname, "segments%s.npy" % suffix), seg.astype(np.float64))
+
+
 def run_reference(args, rank, world):
     if rank != 0:
         return
@@ -322,6 +343,8 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--frames", type=int, default=N_FRAMES)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step decoded to DIR/*.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -395,14 +418,22 @@ def main():
         L.zb200_result_free(step_device())
     ctx.profile(True)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    last_res = None
     barrier()
     with ClockSampler(local) as clk:
         e0.record(stream)
-        for _ in range(args.steps):
-            L.zb200_result_free(step_device())
+        for i in range(args.steps):
+            res = step_device()
+            if args.dump_outputs and i + 1 == args.steps:
+                last_res = res
+            else:
+                L.zb200_result_free(res)
         e1.record(stream)
         barrier()
     dev_ms = e0.elapsed_time(e1) / args.steps
+    if last_res is not None:
+        dump_outputs(args.dump_outputs, ctx, last_res, n_frames, rank)
+        L.zb200_result_free(last_res)
     prof = ctx.profile_read()
     ctx.profile(False)
     scratch = int(L.zb200_last_scratch_bytes(ctx.h))
@@ -479,7 +510,7 @@ def main():
     for _ in range(2):
         L.zb200_result_free(step_compress())
     ce0, ce1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    csteps = max(2, args.steps // 2)
+    csteps = args.steps
     barrier()
     ce0.record(stream)
     for _ in range(csteps):

@@ -721,7 +721,21 @@ static int compress_common(zb200_ctx* ctx, const void* src_base, const zb200_seg
     unsigned long long* const d_progress = (unsigned long long*)(d_counter + 4);
     bool const overlap_upload = up_bytes != 0 && nj != 0 && ctx->h_progress != nullptr;
     if (up_bytes && !overlap_upload) CK(cudaMemcpyAsync(ctx->src.p, up_src, up_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    if (overlap_upload) { CK(cudaEventRecord(ctx->chunk_ev[0], ctx->stream)); CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->chunk_ev[0], 0)); }
+    if (overlap_upload) {
+        // The whole upload is queued BEFORE the compress kernel is launched: the kernel spins until the bytes it needs
+        // have landed, so once it runs, its progress must not depend on this thread reaching further API calls (another
+        // thread's cudaFree on the same device, say, can hold those back until the kernel ends).
+        CK(cudaEventRecord(ctx->chunk_ev[0], ctx->stream)); CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->chunk_ev[0], 0));
+        // <= 48 chunks of >= 4 MiB; after each chunk the copy engine also writes the new byte count next to the work counter
+        u64 chunk = (up_bytes + 47) / 48; if (chunk < ((u64)4 << 20)) chunk = (u64)4 << 20; chunk = (chunk + 255) & ~(u64)255;
+        u32 k = 0;
+        for (u64 pos = 0; pos < up_bytes; pos += chunk, k++) {
+            u64 const len = up_bytes - pos < chunk ? up_bytes - pos : chunk;
+            CK(cudaMemcpyAsync((u8*)ctx->src.p + pos, up_src + pos, len, cudaMemcpyHostToDevice, ctx->copy_stream));
+            ctx->h_progress[k] = pos + len;
+            CK(cudaMemcpyAsync(d_progress, &ctx->h_progress[k], sizeof(unsigned long long), cudaMemcpyHostToDevice, ctx->copy_stream));
+        }
+    }
     ctx->last_compress_kernel = recs_kernel ? "zb_compress_recs" : (smem_kernel ? "zb_compress_smem" : "zb_compress_blocks");
     if (recs_kernel) { KSpan s(ctx, ZB200_K_COMPRESS);
       zb_launch_compress_recs(d_src, ctx->jobs.p, (u32)nj, ctas, ctx->slots.as<u8>(), slot_bytes, ctx->bouts.p, d_counter,
@@ -736,15 +750,6 @@ static int compress_common(zb200_ctx* ctx, const void* src_base, const zb200_seg
                                 (dict && dict->c_D && dict->dev.has_entropy) ? (const void*)dict->d_digest : nullptr, dict ? dict->d_cct : nullptr,
                                 overlap_upload ? d_progress : nullptr, up_bytes, d_upstatus, P.level >= 4 ? 1 : 0, max_block <= zb_encode_small_max() ? 1 : 0, ctx->stream); }
     if (overlap_upload) {
-        // <= 48 chunks of >= 4 MiB; after each chunk the copy engine also writes the new byte count next to the work counter
-        u64 chunk = (up_bytes + 47) / 48; if (chunk < ((u64)4 << 20)) chunk = (u64)4 << 20; chunk = (chunk + 255) & ~(u64)255;
-        u32 k = 0;
-        for (u64 pos = 0; pos < up_bytes; pos += chunk, k++) {
-            u64 const len = up_bytes - pos < chunk ? up_bytes - pos : chunk;
-            CK(cudaMemcpyAsync((u8*)ctx->src.p + pos, up_src + pos, len, cudaMemcpyHostToDevice, ctx->copy_stream));
-            ctx->h_progress[k] = pos + len;
-            CK(cudaMemcpyAsync(d_progress, &ctx->h_progress[k], sizeof(unsigned long long), cudaMemcpyHostToDevice, ctx->copy_stream));
-        }
         // the layout kernels read the input again (raw blocks): they wait for the whole upload, whatever order the segments came in
         CK(cudaEventRecord(ctx->chunk_ev[1], ctx->copy_stream)); CK(cudaStreamWaitEvent(ctx->stream, ctx->chunk_ev[1], 0));
     }
